@@ -4,6 +4,7 @@
 
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also writes x and r of the last timed sweep
 
 A "step" is one sweep: BLOCK block steps, each reading the column block A_m for the block
 gradient A_m^T r and again for A_m D (prox, line search, error and updates fused).  The
@@ -523,6 +524,33 @@ def time_sweeps(cx, cal, b, mu, BLOCK, steps, warmup, single_launch=False, sampl
     return ms / steps, clocks
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(cx, cal, BLOCK, directory):
+    """write the solution x and the residual r = Ax - b, as the last timed sweep left them on the device,
+    to directory/x.npy and directory/r.npy (float64).  Several GPUs: x is gathered into global column
+    order and rank 0 writes.  An array larger than its share of DUMP_BYTES is replaced by a fixed sample
+    of its entries (sorted indices drawn by np.random.RandomState(0)), the same for every run of a shape."""
+    from convex_optimization_b200 import _lib
+    x = np.empty(cal.MAT_WIDTH_ALL)
+    r = np.empty(cal.MAT_HEIGHT)
+    _lib.check(cal._lib.b200l_get_x(cal.ctx, _lib.dptr(x)))
+    _lib.check(cal._lib.b200l_get_r(cal.ctx, _lib.dptr(r)))
+    if cx.world > 1:
+        from convex_optimization_b200 import distributed as dd
+        x = dd.gather_x(x, BLOCK).reshape(-1)
+    if cx.rank != 0:
+        return
+    os.makedirs(directory, exist_ok=True)
+    outputs = {"x": x, "r": r}
+    for name, a in outputs.items():
+        limit = DUMP_BYTES // len(outputs) // a.itemsize
+        if a.size > limit:
+            a = a[np.sort(np.random.RandomState(0).choice(a.size, limit, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def roofline_record(cx, cfg, layout, ms_per_sweep, sweeps_per_launch, traffic_key, l2_bytes):
     N, K, BLOCK = cfg["N"], cfg["K"], cfg["BLOCK"]
     s = 4 if cfg["dtype"] == "float" else 8
@@ -684,6 +712,8 @@ def main_gpu(args):
     single_launch = args.single_launch or world > 1
     ms_per_step, clocks = time_sweeps(cx, cal, b, mu, BLOCK, args.steps, args.warmup, single_launch,
                                       sampler if rank == 0 else None)
+    if args.dump_outputs:
+        dump_outputs(cx, cal, BLOCK, args.dump_outputs)
     value = world * 1e3 / ms_per_step
     sweeps_per_launch = args.steps if single_launch else 1
     n_launches = args.steps // sweeps_per_launch
@@ -835,7 +865,15 @@ def main():
     ap.add_argument("--shape", default="", help="diagnostics: N,K,BLOCK[,float|double] instead of a named config")
     ap.add_argument("--config", default="c2", choices=["c2", "c3", "c4shard"],
                     help="c2 is the bench workload; the others appear as sub-records of the default run")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed sweeps, write x and r = Ax - b of the last one as DIR/x.npy and DIR/r.npy "
+                         "(float64, at most 64 MB in all); the instance depends only on the arguments, so two builds "
+                         "can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return main_reference(args)

@@ -1,8 +1,10 @@
 """The reference's own drivers, UNMODIFIED, against this package (SURVEY.md section 8b / VERDICT round 1
 "missing" 1): ``cpu_vs_gpu.py`` and ``compare.py`` run through the drop-in directory
 (convex_optimization_b200/dropin: flat module names + pycuda / skcuda shims + a headless matplotlib
-fallback).  The scripts come from oracle/_ref (an unmodified copy made by oracle/make_ref.py, which
-travels to the GPU box) or from the reference tree itself; without either the tests skip."""
+fallback).  The scripts come from oracle/_ref, an unmodified copy of the reference's files that
+oracle/make_ref.py makes from a checkout of the reference; the reference's sources are not part of
+this repository, so without that copy the tests skip."""
+import json
 import os
 import subprocess
 import sys
@@ -12,15 +14,15 @@ import pytest
 
 from conftest import ROOT, load_golden
 
-REF_DIRS = [os.path.join(ROOT, "oracle", "_ref"), "/root/reference"]
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def ref_script(name):
-    for d in REF_DIRS:
-        p = os.path.join(d, name)
-        if os.path.exists(p):
-            return p
-    pytest.skip("neither oracle/_ref nor the reference tree holds %s" % name)
+    p = os.path.join(REF_DIR, name)
+    if not os.path.exists(p):
+        pytest.skip("oracle/_ref does not hold %s (run oracle/make_ref.py with B200L_REFERENCE set to a "
+                    "checkout of the reference)" % name)
+    return p
 
 
 def run_dropin(script, env_extra, timeout=600):
@@ -36,9 +38,11 @@ def test_oracle_ref_copies_are_unmodified():
     if not make_ref.available():
         pytest.skip("oracle/_ref is not populated")
     assert make_ref.check()
-    if os.path.isdir(make_ref.reference_dir()):
+    with open(os.path.join(make_ref.DEST, make_ref.MANIFEST)) as f:
+        source = json.load(f)["source"]             # the checkout the copies were made from
+    if os.path.isdir(source):
         for name in make_ref.FILES:
-            with open(os.path.join(make_ref.reference_dir(), name), "rb") as f1, \
+            with open(os.path.join(source, name), "rb") as f1, \
                     open(os.path.join(make_ref.DEST, name), "rb") as f2:
                 assert f1.read() == f2.read(), name
 

@@ -130,3 +130,63 @@ def test_bench_reference_arm_prints_the_contract_line(monkeypatch, capsys):
     monkeypatch.setenv("RANK", "1")
     assert bench.main_reference(args) == 0
     assert capsys.readouterr().out == ""
+
+
+def test_bench_dump_outputs_writes_x_and_r_within_the_budget(monkeypatch, tmp_path):
+    """bench.py --dump-outputs: x and r as float64 .npy; past the byte budget a fixed sample of the entries"""
+    import types
+    import bench
+    N, K = 300, 4000
+    x_dev, r_dev = np.arange(K) * 0.5, -np.arange(N) - 1.0
+
+    def copy_out(src):
+        def get(ctx, ptr):
+            np.ctypeslib.as_array(ptr, shape=(src.size,))[:] = src
+            return 0
+        return get
+    lib = types.SimpleNamespace(b200l_get_x=copy_out(x_dev), b200l_get_r=copy_out(r_dev))
+    cal = types.SimpleNamespace(_lib=lib, ctx=None, MAT_WIDTH_ALL=K, MAT_HEIGHT=N)
+    cx = types.SimpleNamespace(world=1, rank=0)
+    bench.dump_outputs(cx, cal, 4, str(tmp_path / "full"))
+    x, r = np.load(tmp_path / "full" / "x.npy"), np.load(tmp_path / "full" / "r.npy")
+    assert x.dtype == r.dtype == np.float64
+    assert np.array_equal(x, x_dev) and np.array_equal(r, r_dev)
+    # several GPUs: x is gathered over the ranks and only rank 0 writes
+    from convex_optimization_b200 import distributed as dd
+    monkeypatch.setattr(dd, "gather_x", lambda x_local, BLOCK: np.concatenate([x_local, x_local + K]).reshape(-1, 1))
+    for rank in (1, 0):
+        bench.dump_outputs(types.SimpleNamespace(world=2, rank=rank), cal, 4, str(tmp_path / ("rank%d" % rank)))
+    assert not (tmp_path / "rank1").exists()
+    assert np.array_equal(np.load(tmp_path / "rank0" / "x.npy"), np.concatenate([x_dev, x_dev + K]))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 8 * 1000)            # x over its share, r within it
+    for run in ("a", "b"):
+        bench.dump_outputs(cx, cal, 4, str(tmp_path / run))
+    xa, xb = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "b" / "x.npy")
+    assert xa.size == 1000 and np.array_equal(xa, xb)                 # the same sample every run
+    assert np.all(np.diff(xa) > 0) and np.all(np.isin(xa, x_dev))     # entries of x, in index order
+    assert np.array_equal(np.load(tmp_path / "a" / "r.npy"), r_dev)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_from_run_to_run(tmp_path):
+    """bench.py --dump-outputs on the CUDA path: two runs with the same arguments write the same x and r
+    (the fused kernel is bitwise deterministic), and one more timed sweep changes them"""
+    import json
+    import subprocess
+    import sys
+
+    def run(tag, steps):
+        out = tmp_path / tag
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--small", "--quick", "--no-cpu", "--no-parity",
+               "--eps", "0", "--steps", str(steps), "--warmup", "3", "--dump-outputs", str(out)]
+        proc = subprocess.run(cmd, cwd=str(tmp_path), capture_output=True, text=True, timeout=600)
+        assert proc.returncode == 0, proc.stdout[-2000:] + proc.stderr[-2000:]
+        assert json.loads(proc.stdout.strip().splitlines()[-1])["steps"] == steps
+        return np.load(out / "x.npy"), np.load(out / "r.npy")
+    xa, ra = run("a", 2)
+    xb, rb = run("b", 2)
+    xc, _ = run("c", 3)
+    assert xa.shape == (20000,) and ra.shape == (2000,) and xa.dtype == ra.dtype == np.float64
+    assert np.count_nonzero(xa) > 0 and np.all(np.isfinite(ra))
+    assert np.array_equal(xa, xb) and np.array_equal(ra, rb)
+    assert not np.array_equal(xc, xa)
