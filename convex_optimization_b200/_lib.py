@@ -12,7 +12,7 @@ import sys
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_PKG)
-# B200L_LIB selects another build of the same source (diagnostics, e.g. -DB200L_LEAN)
+# B200L_LIB selects another build of the library (e.g. an older one, to compare outputs)
 LIB_PATH = os.environ.get("B200L_LIB") or os.path.join(_PKG, "libb200lasso.so")
 SRC = os.path.join(_PKG, "csrc", "b200lasso.cu")
 INCLUDE = os.path.join(_ROOT, "include")

@@ -30,10 +30,6 @@
 
 #include "b200lasso.h"
 
-#ifndef B200L_MAX_WORLD
-#define B200L_MAX_WORLD 8
-#endif
-
 // ------------------------------------------------------------------------------------
 // error plumbing
 // ------------------------------------------------------------------------------------
@@ -292,10 +288,10 @@ template <> struct LLW<double> {
 
 constexpr int NTTRACE = 96;        // per-tile stamps: 6 groups of 16 (see b200lasso.h)
 constexpr int NTRACE = 16;         // time stamps per CTA and step of b200l_run_traced
-#ifndef B200L_P1_UNROLL
-#define B200L_P1_UNROLL 1
-#endif
-constexpr int P1U = B200L_P1_UNROLL;   // row quads of pass 1 in flight per thread
+// b200l_debug_flags: bits 0-2 switch parts of the fused kernel off to time the rest (1 exchange waits,
+// 2 pass-1 math, 4 pass-2 math; the diagnostic instantiation, results meaningless), bit 18 keeps the
+// step-wise mat-vecs on the load-batch kernels (results valid)
+constexpr int32_t DBG_KNOCKOUTS = 7, DBG_LOAD_BATCH = 262144;
 constexpr int NB = 8;              // exchange words a thread keeps in flight per round trip
 constexpr int GMAX = 160;          // largest grid (sizes the acknowledgement words of the step-D exchange)
 
@@ -343,18 +339,17 @@ struct RunParams {
     unsigned long long *trace;  // optional [G][nsteps][NTRACE] phase time stamps (ns since start)
     unsigned long long *ttrace; // optional [G][nsteps][NTTRACE] per-tile time stamps (absolute ns)
     uint32_t tag_base;
-    int32_t dbg;          // diagnostics only: 1 skip exchange waits, 2 skip pass-1 math, 4 skip pass-2 math
     unsigned long long wait_limit_ns;
     // geometry
-    int32_t TR, S, slot_bytes, cs, cs_shift, nrg, ncg, rows_pad, rows_max_, inflight, l2_ahead;
+    int32_t TR, S, slot_bytes, cs, cs_shift, nrg, ncg, rows_pad, rows_max_, l2_ahead;
     // multi-GPU: rank `rank` of `world` holds column slice `rank` of every block; peer[r] is the
     // q-inbox of rank r: [2 parities][G CTAs][world sources][qw] words (peer[rank] is local)
-    int32_t xmode;            // multi-GPU send side: 0 the sender warp sends finished pass-2 tiles, 1 the lane that finishes a row sends it
-    int32_t world, rank, qw, tile_sends; // qw: words per rank in a cell; tile_sends: plan for xmode 0
+    int32_t tile_sends;       // multi-GPU send side: 1 the sender warp sends finished pass-2 tiles, 0 the lane that finishes a row sends it
+    int32_t world, rank, qw;  // qw: words per rank in a cell
     ulonglong2 *peer[B200L_MAX_WORLD];
     ulonglong2 *mc;           // multicast mapping of all ranks' inboxes (NVLS) or NULL
     int32_t direct_pub;       // partial gradients are published from registers (one row group)
-    int32_t gate_mode;        // 0: re-stream freely, 1/2/3: after inbox fetch issued / gather done / D fetch issued
+    int32_t dbg;              // diagnostics only: 1 skip exchange waits, 2 skip pass-1 math, 4 skip pass-2 math
     int32_t gate2_tiles;      // > 0: only this many pass-2 tiles are staged before the step-D gather is complete
     // transposed layout: a tile is TJ block columns x BX residual entries of this CTA
     // (BX/V odd: conflict-free 16-byte reads with lanes on consecutive columns)
@@ -587,10 +582,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
     if (wid == NW) {
         // ============================ producer warp ================================
         if (lane == 0) {
-            unsigned long long k = 0, kd = 0;   // tiles issued / tiles known to have landed
+            unsigned long long k = 0;   // tiles issued
             Cursor cur{0, 1u};   // waits on "empty" with the inverted parity
-            Cursor dcur{0, 0u};  // oldest tile not yet known to have landed
-            const unsigned long long max_inflight = (unsigned long long)p.inflight;
             volatile int *stopf = &ctl->stop;
             bool live = true;
             int mc = (int)(p.step0 % p.nblocks);
@@ -608,8 +601,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                 }
                 const int ym = m * p.w, yn = (p.order ? (step + 1 < p.nsteps ? p.order[step + 1] : 0) : mc) * p.w;
                 for (int pass = 0; pass < 2 && live; ++pass) {
-                    // the re-stream for pass 2 can be held back (gate) behind the consumers' exchange
-                    if (pass == 1 && p.gate_mode) {
+                    // the re-stream for pass 2 waits (gate) until this CTA's gather is complete: issued
+                    // earlier, the tiles queue the gather's loads behind them on the L2 link
+                    if (pass == 1) {
                         while (*(volatile long long *)&ctl->gate <= step) {
                             if (*stopf) { live = false; break; }
                             __nanosleep(64);
@@ -623,17 +617,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                             }
                             if (!live) break;
                         }
-                        // pacing: a bounded number of bulk copies in flight
-                        while (k - kd >= max_inflight) {
-                            if (mbar_try_wait(full + dcur.slot, dcur.phase)) {
-                                dcur.advance(S);
-                                ++kd;
-                            } else if (*stopf) {
-                                live = false;
-                                break;
-                            }
-                        }
-                        if (!live) break;
                         while (!mbar_try_wait(empty + cur.slot, cur.phase)) {
                             if (*stopf) { live = false; break; }
                         }
@@ -670,7 +653,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
         // with a pass-2 tile: consecutive lanes = consecutive words (whole NVLink packets), and
         // the peer stores stay out of the inner loop of pass 2.  (TRANS, or more tiles than
         // counters: the consumers send their rows themselves.)
-        if (WORLD > 1 && p.xmode == 0) {
+        if (WORLD > 1 && p.tile_sends) {
             Waiter hw{p.abort_flag, &ctl->abort, p.wait_limit_ns, 0u, 0ull, p.state + 4, 0};
             bool live = true;
             for (long long hs = 0; live; ++hs) {
@@ -784,8 +767,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                             // consumers send their rows themselves
                             const long long pd = *(volatile long long *)&ctl->p2done;
                             const long long orw = *(volatile long long *)&ctl->own_rows;
-                            int mine_n = p.xmode == 0 ? ((orw >> 32) == hs + 1 ? (int)(orw & 0x7fffffff) : 0)
-                                                      : (pd > hs ? rows_c : 0);
+                            int mine_n = p.tile_sends ? ((orw >> 32) == hs + 1 ? (int)(orw & 0x7fffffff) : 0)
+                                                   : (pd > hs ? rows_c : 0);
                             mine_n = __reduce_min_sync(0xffffffffu, mine_n);
                             if (mine_n > own_rows) {
                                 own_rows = mine_n;
@@ -1102,7 +1085,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                             // there is stale (possibly words of an exchange fetch, i.e. NaN bit
                             // patterns), so the last row of the tile is read in its place
                             const int nquad = (rows_t + 3) >> 2;
-#pragma unroll(P1U)
+#pragma unroll 1
                             for (int q4 = rg; q4 < nquad; q4 += nrg) {
                                 T rv[4], qv[4];
                                 load4(rTt + 4 * q4, rv);
@@ -1180,11 +1163,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                     }
                 }
             }
-#ifdef B200L_PUBBAR
-            cbar();
-#else
             if (!p.direct_pub && !drain) cbar();       // the row-group partials in shared memory are complete
-#endif
             // ---------------- publish: one message of MW words per reader -------------------
             // the partial gradient (g_r, g_q) of the cs columns that reader owns: MW = cs * WPC
             // words, a power of two (C2: 8 words = one 128-byte line per reader).  My four
@@ -1218,7 +1197,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                     }
                 }
             }
-            if (tid == 0 && p.gate_mode == 1) *(volatile long long *)&ctl->gate = step + 1;
             if (trace && !drain) trace[step * NTRACE + 2] = tstamp() - c_start;
 
             // ---------------- gather -------------------------------------------------------
@@ -1307,7 +1285,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                     }
                 }
             }
-            if (tid == 0 && p.gate_mode == 2) *(volatile long long *)&ctl->gate = step + 1;
+            if (tid == 0) *(volatile long long *)&ctl->gate = step + 1;   // the producer may re-stream the slab
             if (trace && !drain) trace[step * NTRACE + 3] = trace[step * NTRACE + 4] = tstamp() - c_start;
 
             // ---------------- resolve the pending step: error, stop rule, gamma ---------
@@ -1399,7 +1377,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
             if (!drain) {
                 const int dwords = ld / p.dpw;
                 const int dtot = p.ackbase + 2 * (G - p.nown);    // D words + acknowledgements
-                if (tid == 0 && p.gate_mode == 3) *(volatile long long *)&ctl->gate = step + 1;
 #pragma unroll 1
                 for (int base = tid; base < dtot; base += NTC * NB) {
                     ulonglong2 v[NB];
@@ -1489,7 +1466,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                 }
             };
             if (WORLD > 1 && tid == 0) {   // my l1 / err terms of this step travel with the rows
-                if (p.xmode == 1) {        // (otherwise the sender warp sends them)
+                if (!p.tile_sends) {       // (otherwise the sender warp sends them)
                     send_row(rows_c, ctl->sp[2]);
                     send_row(rows_c + 1, ctl->sp[3]);
                 }
@@ -1555,14 +1532,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) lasso_fused(const RunParams p, co
                     if (row_a >= 0 && (lane & 15) == 0 && (two || lane == 0)) {
                         const int row = row_a + (lane >> 4) * NW;
                         qpart[row] = (double)qs;
-                        if (p.xmode == 1) send_row(row, (double)qs);
+                        if (!p.tile_sends) send_row(row, (double)qs);
                     }
                 };
                 if (trace) trace[step * NTRACE + 14] = tstamp() - c_start;
                 // multi-GPU: the sender warp sends a tile's rows to the peers when all NW warps have
                 // counted it
                 auto count_tile = [&](int tile_idx) {
-                    if (WORLD > 1 && p.xmode == 0) {
+                    if (WORLD > 1 && p.tile_sends) {
                         __syncwarp();
                         if (lane == 0) {
                             __threadfence_block();
@@ -2351,7 +2328,7 @@ struct b200l_ctx {
     int have_problem, have_diag;
     cudaEvent_t ev0, ev1;
     // tuning
-    int32_t slot_target, max_inflight, dbg;
+    int32_t slot_target, dbg;
     CUtensorMap tmap;             // transposed layout only
     int tmap_valid;
     // multi-GPU
@@ -2441,7 +2418,6 @@ extern "C" int b200l_ctx_create(b200l_ctx **out, int dtype, int layout, int64_t 
     c->smem_optin = (int)prop.sharedMemPerBlockOptin;
     c->l2_bytes = prop.l2CacheSize;
     c->slot_target = 0;
-    c->max_inflight = 0;
     c->wait_limit_ns = 5000000000ULL;
     c->world = 1;
     c->rank = 0;
@@ -2615,7 +2591,7 @@ static int rowdot_stream_try(b200l_ctx *c, const T *Ablk, int64_t M, int ncols, 
                              double *out, int accumulate, bool *done) {
     constexpr int V = VT<T>::V;
     *done = false;
-    if (c->dbg & 262144) return 0;                               // (load-batch kernels only: tests, comparisons)
+    if (c->dbg & DBG_LOAD_BATCH) return 0;                       // (load-batch kernels only: tests, comparisons)
     if ((int64_t)M * ncols * (int64_t)sizeof(T) < MS_MIN_BYTES || M < 2 * c->sm_count) return 0;
     const int ncg = ncols / V;
     MsParams p;
@@ -2973,8 +2949,11 @@ extern "C" int b200l_set_diag(b200l_ctx *c, const double *d_host) {
 // ------------------------------------------------------------------------------------
 extern "C" int b200l_set_tuning(b200l_ctx *c, int32_t slot_bytes_target, int32_t max_inflight_tiles) {
     if (!c) return fail("ctx is NULL");
+    // the ring's empty barriers already cap the copies in flight at the ring size; no other cap is offered
+    if (max_inflight_tiles != 0)
+        return fail("max_inflight_tiles=%d: only 0 (as many bulk copies in flight as ring slots) is supported",
+                    max_inflight_tiles);
     c->slot_target = slot_bytes_target > 0 ? slot_bytes_target : 0;   // 0: chosen per shape
-    c->max_inflight = max_inflight_tiles;
     c->geo_valid = 0;
     return 0;
 }
@@ -3067,7 +3046,10 @@ static int plan_geometry(b200l_ctx *c) {
     int cs = 1, cs_shift = 0;
     while (cs * G < ld) { cs *= 2; ++cs_shift; }
     if (cs > MAX_CS) return fail("internal: slice width %d > %d", cs, MAX_CS);
-    const int direct_pre = (!trans && nrg == 1 && cs * (es / 4) >= 4 && !(c->dbg & 128)) ? 1 : 0;
+    // the partial gradient goes out straight from registers when every thread holds complete column sums
+    // (one row group) and a column group (4 words, two 256-bit stores) fits one message of cs * es / 4 words;
+    // otherwise the row groups are combined through shared memory first
+    const int direct = (trans || (nrg == 1 && cs * (es / 4) >= 4)) ? 1 : 0;
     int slot_bytes = trans ? 0 : (int)round_up((int64_t)TR * rowbytes, 128);
     int rows_pad = trans ? 0 : (int)round_up(std::max(rows_max, 1), std::max(TR, 8));
 
@@ -3082,7 +3064,7 @@ static int plan_geometry(b200l_ctx *c) {
         const int o_qT = take(rows_pad * es);
         // the step D (written after the gather, read in pass 2) overlays the row-group
         // partials (written after pass 1, read before the gather): two barriers apart
-        const int o_redT = take(trans ? nt_t * TJ * es : (direct_pre ? ld * es : nrg * 2 * ld * es));
+        const int o_redT = take(trans ? nt_t * TJ * es : (direct ? ld * es : nrg * 2 * ld * es));
         const int o_red2 = take(trans ? nparts * BX * es : 16);
         const int o_delta = o_redT;
         const int o_red = take(NTC * 16);                          // gather partials per thread
@@ -3094,16 +3076,6 @@ static int plan_geometry(b200l_ctx *c) {
             out->off_rT = o_rT; out->off_qT = o_qT; out->off_delta = o_delta; out->off_redT = o_redT;
             out->off_red = o_red; out->off_small = o_small; out->off_qpart = o_qpart;
             out->off_red2 = o_red2; out->off_tilecnt = o_tilecnt;
-            // multi-GPU send side: the sender warp sends the rows of a pass-2 tile when the
-            // consumer warps are done with it (row-major, up to 128 tiles); otherwise the lane that
-            // finishes a row stores it to every peer itself (also forced by dbg bit 8)
-            const int nt_plan = trans ? nt_t : (rows_max + TR - 1) / TR;
-            // (with a single peer the consumer lanes send their rows themselves: +1 % on 2 GPUs.  On 8 GPUs
-            // the sender warp wins even when a multicast mapping makes it one store per row -- measured per
-            // block step: sender warp + multimem 18.9 us, sender warp + 7 unicast stores 19.2, consumer lanes
-            // + multimem 20.2, consumer lanes + unicast 23.9)
-            const bool one_store = c->world == 2 && !(c->dbg & 512);
-            out->tile_sends = (c->world > 1 && !trans && nt_plan <= 128 && !(c->dbg & 256) && !one_store) ? 1 : 0;
         }
     };
     if (trans) {
@@ -3168,16 +3140,21 @@ static int plan_geometry(b200l_ctx *c) {
     c->grid = G;
     c->cpt = cpt;
     c->nt_max = nt_max;
+    // multi-GPU send side: the sender warp sends the rows of a pass-2 tile when the consumer warps are
+    // done with it (row-major, up to 128 tiles: its counters); otherwise the lane that finishes a row
+    // stores it to every peer itself.  With a single peer the consumer lanes win: +1 % on 2 GPUs.  On 8
+    // GPUs the sender warp wins even when a multicast mapping makes it one store per row -- measured per
+    // block step: sender warp + multimem 18.9 us, sender warp + 7 unicast stores 19.2, consumer lanes
+    // + multimem 20.2, consumer lanes + unicast 23.9
+    g.tile_sends = (c->world > 2 && !trans && nt_max <= 128) ? 1 : 0;
     // exchange geometry
     const int wpc = es / 4;
     // message = the cs columns of one reader, cs * wpc words: a power of two that divides NTC
-    // (thread = word in the gather).  Publishing from registers needs complete column sums per
-    // thread (one row group) and a column group (4 words, two 256-bit stores) inside one message
+    // (thread = word in the gather)
     const int mw = cs * wpc;
     int mw_shift = 0;
     while ((1 << mw_shift) < mw) ++mw_shift;
     if ((1 << mw_shift) != mw || mw > NTC) return fail("internal: message width %d", mw);
-    const int direct = trans ? 1 : ((nrg == 1 && mw >= 4 && !(c->dbg & 128)) ? 1 : 0);
     const int nown = (ld + cs - 1) / cs;                 // CTAs that own at least one column
     g.TR = TR; g.S = S; g.slot_bytes = slot_bytes; g.cs = cs; g.cs_shift = cs_shift;
     g.ring_bytes = S * slot_bytes;
@@ -3191,24 +3168,19 @@ static int plan_geometry(b200l_ctx *c) {
     g.BX = BX; g.BXV = BXV; g.TJ = TJ; g.nparts = nparts; g.nt_t = nt_t;
     g.NBX = NBX; g.BXb = BXVb * V; g.BXVb = BXVb; g.P1 = P1;
     c->tmap_valid = 0;
-    g.inflight = c->max_inflight > 0 ? std::min(c->max_inflight, S) : S;
     // HBM one block ahead through L2 only pays when this block (re-read by pass 2) and the next
     // one fit in L2 together; for larger blocks the prefetched lines would be evicted before use
     const int64_t block_bytes = (int64_t)c->brows * c->ld * es;
-    g.l2_ahead = ((c->dbg & 8) || 2 * block_bytes > (int64_t)c->l2_bytes * 3 / 4) ? 0 : 1;
-    // when the producer may start re-streaming the slab for pass 2, so that the tiles are staged in
-    // the ring while the rest of the exchange runs: 2 = once this CTA's gather is complete (default;
-    // measured on C2: 810 sweeps/s), 1 = once it has published its partial gradient (788), 0 = at once
-    // (the gather's loads queue behind the tiles on the L2 link: 660-700), 3 = after the prox
-    // (diagnostics: dbg bits 5-6 = 1 / 2 / 3 select modes 0 / 1 / 3)
-    const int gm = (c->dbg >> 5) & 3;
-    g.gate_mode = gm == 0 ? 2 : (gm == 1 ? 0 : (gm == 2 ? 1 : 3));
-    // ... and the last ring slot is only filled once the step-D gather is complete: with all four slots in flight
+    g.l2_ahead = 2 * block_bytes > (int64_t)c->l2_bytes * 3 / 4 ? 0 : 1;
+    // The producer starts re-streaming the slab for pass 2 once this CTA's gather is complete (the gate), so
+    // that the tiles are staged in the ring while the rest of the exchange runs (measured on C2: 810 sweeps/s;
+    // from the publish of the partial gradient on 788; at once 660-700, the gather's loads queue behind the
+    // tiles on the L2 link).  The last ring slot is only filled once the step-D gather is complete (the second
+    // gate, gate2_tiles early tiles): with all four slots in flight
     // the gather's polls queue behind one more tile on the L2 link (measured on C2, one GPU, same box: 832.5 vs
     // 822.5 sweeps/s; holding back two slots 812, three 760).  Blocks that stay in L2, one GPU, row-major, at
-    // least four slots; dbg bits 20-22 = 1..6 set the number of early tiles, 7 switches the second gate off.
-    const int g2 = (c->dbg >> 20) & 7;
-    g.gate2_tiles = g2 == 7 ? 0 : (g2 ? g2 : ((l2_resident && !trans && c->world == 1 && S >= 4) ? S - 1 : 0));
+    // least four slots.
+    g.gate2_tiles = (l2_resident && !trans && c->world == 1 && S >= 4) ? S - 1 : 0;
 
     // inboxes of the partial block gradients: [G readers][G writers][cs][WPC] LL words
     const size_t need = (size_t)G * G * mw * 16;
@@ -3313,11 +3285,8 @@ static int launch_fused(b200l_ctx *c, const int32_t *order_host, int64_t nsteps,
     p.world = c->world;
     p.rank = c->rank;
     p.qw = c->world > 1 ? (int32_t)round_up(c->geo.rows_max_ + 2, 2) : 0;
-    p.tile_sends = c->geo.tile_sends;
-    p.xmode = c->geo.tile_sends ? 0 : 1;
     for (int r = 0; r < B200L_MAX_WORLD; ++r) p.peer[r] = c->peer[r];
     p.mc = c->world > 1 ? c->mc : nullptr;
-    p.dbg = c->dbg;
 
     if (c->world > 1)
         for (int r = 0; r < c->world; ++r)
@@ -3325,8 +3294,9 @@ static int launch_fused(b200l_ctx *c, const int32_t *order_host, int64_t nsteps,
                 return fail("multi-GPU run: the inbox of rank %d is not mapped (b200l_comm_connect has not "
                             "completed on this context)", r);
     if (c->layout == B200L_TRANSPOSED && !c->tmap_valid && make_tensor_map(c)) return 1;
-    const bool diag = trace_dev != nullptr || ttrace_dev != nullptr || (c->dbg & 7) != 0;
-    fused_fn fn = ctx_kernel(c, diag ? 2 : ((c->world > 1 || (c->dbg & 4096)) ? 1 : 0));   // (dbg 4096: mode 1 on one GPU, to time the variant)
+    p.dbg = c->dbg & DBG_KNOCKOUTS;
+    const bool diag = trace_dev != nullptr || ttrace_dev != nullptr || p.dbg != 0;
+    fused_fn fn = ctx_kernel(c, diag ? 2 : (c->world > 1 ? 1 : 0));
     void *args[] = {(void *)&p, (void *)&c->tmap};
     if (timed) CK(cudaEventRecord(c->ev0, c->stream));
     CK(cudaLaunchCooperativeKernel((const void *)fn, dim3(c->grid), dim3(NTHREADS), args,
@@ -3435,12 +3405,13 @@ extern "C" int b200l_set_wait_limit(b200l_ctx *c, double seconds) {
     return 0;
 }
 
-// diagnostics only (tools/trace_fused.py): switches parts of the fused kernel off to time
-// the rest; results of a run with flags != 0 are meaningless
+// diagnostics (see DBG_KNOCKOUTS, DBG_LOAD_BATCH)
 extern "C" int b200l_debug_flags(b200l_ctx *c, int32_t flags) {
     if (!c) return fail("ctx is NULL");
+    if (flags & ~(DBG_KNOCKOUTS | DBG_LOAD_BATCH))
+        return fail("debug flags 0x%x: only bits 0-2 (1, 2, 4: knock-outs) and bit 18 (262144: load-batch "
+                    "mat-vecs) are accepted", (unsigned)flags);
     c->dbg = flags;
-    c->geo_valid = 0;
     return 0;
 }
 

@@ -134,7 +134,8 @@ int b200l_run(b200l_ctx *ctx, const int32_t *order_host, int64_t nsteps, double 
 int b200l_run_config(b200l_ctx *ctx, int32_t *grid, int32_t *threads, int32_t *smem_bytes,
                      int32_t *tile_rows, int32_t *ring_slots, int32_t *tiles_per_slab);
 /* tunables: ring slot bytes target (0 = default: 48 KiB when a block stays in L2 between the two
- * passes, else 64 KiB), bulk copies in flight per CTA (0 = ring size) */
+ * passes, else 64 KiB).  max_inflight_tiles must be 0: a CTA keeps as many bulk copies in flight as
+ * its ring has slots, and any other value fails. */
 int b200l_set_tuning(b200l_ctx *ctx, int32_t slot_bytes_target, int32_t max_inflight_tiles);
 
 /* Diagnostics of the hot path.  run_traced runs `nsteps` unbounded steps (cyclic order,
@@ -161,7 +162,8 @@ int b200l_set_wait_limit(b200l_ctx *ctx, double seconds);
 /* diagnostics only: bit 0 skips the exchange waits, bit 1 the pass-1 arithmetic, bit 2 the
  * pass-2 arithmetic of the fused kernel, to time the remaining parts.  Results are invalid.
  * Bit 18 (262144) is the one flag with valid results: the step-wise mat-vecs then always use the
- * load-batch kernels instead of the TMA-streamed one (tests cover both). */
+ * load-batch kernels instead of the TMA-streamed one (tests cover both).  flags with any other
+ * bit set fail and leave the previous flags in place. */
 int b200l_debug_flags(b200l_ctx *ctx, int32_t flags);
 
 /* -- synthetic instances on the device (reference recipe: parameters.py:20-28) ---------

@@ -284,6 +284,17 @@ def test_error_paths():
         _lib.check(cal._lib.b200l_run(cal.ctx, None, 4, 0.1, -1.0, None, None, None, None, None))
     with pytest.raises(_lib.B200LassoError):
         cal.mat_tMulVec_DiffSize(np.zeros((4, 1)), 7, np.zeros((8, 1)))
+    # debug flags: the knock-outs (bits 0-2) and the load-batch mat-vecs (bit 18) only; the tuning
+    # call takes a slot size but no cap on the bulk copies in flight
+    for flags in (1, 2, 4, 7, 262144, 262144 | 7, 0):
+        _lib.check(cal._lib.b200l_debug_flags(cal.ctx, flags))
+    for flags in (8, 32, 64, 128, 256, 512, 4096, 1 << 20, 7 << 20, 262144 | 4096, -1):
+        with pytest.raises(_lib.B200LassoError, match="bits 0-2"):
+            _lib.check(cal._lib.b200l_debug_flags(cal.ctx, flags))
+    cal.set_tuning(49152, 0)
+    with pytest.raises(_lib.B200LassoError, match="max_inflight_tiles"):
+        cal.set_tuning(0, 2)
+    cal.set_tuning(0, 0)
     # a block row beyond 32 KiB: the C entry point of the fused kernel refuses it loudly; the solver
     # classes (which accept any block width in the reference) warn and run the step-wise DEVICE path
     # (two library mat-vecs per iteration) -- never a CPU fallback

@@ -29,8 +29,7 @@ def main():
     ap.add_argument("--sweeps", type=int, default=3)
     ap.add_argument("--layout", default="row", choices=["row", "transposed"])
     ap.add_argument("--slot-bytes", type=int, default=0)
-    ap.add_argument("--inflight", type=int, default=0)
-    ap.add_argument("--sweep", default="", help="semicolon list of slot,inflight[,dbg] tuples")
+    ap.add_argument("--sweep", default="", help="semicolon list of slot[,dbg] tuples (dbg: b200l_debug_flags bits 0-2)")
     ap.add_argument("--out", default="")
     ap.add_argument("--raw", default="", help="prefix for raw trace dumps (.npy)")
     ap.add_argument("--tiles", action="store_true", help="per-tile durations of the two passes")
@@ -62,14 +61,14 @@ def main():
     lib, ctx = cal._lib, cal.ctx
     bb = np.ascontiguousarray(b.reshape(-1))
     NT = _lib.NTRACE
-    combos = [(args.slot_bytes, args.inflight, 0)]
+    combos = [(args.slot_bytes, 0)]
     if args.sweep:
         combos = [tuple(int(v) for v in c.split(",")) for c in args.sweep.split(";") if c]
     results = []
     for combo in combos:
-        slot, infl = combo[:2]
-        dbg = combo[2] if len(combo) > 2 else 0
-        cal.set_tuning(slot, infl)
+        slot = combo[0]
+        dbg = combo[1] if len(combo) > 1 else 0
+        cal.set_tuning(slot)
         _lib.check(lib.b200l_debug_flags(ctx, dbg))
         _lib.check(lib.b200l_set_problem(ctx, _lib.dptr(bb)))
         geo = cal.run_config()
@@ -104,7 +103,7 @@ def main():
         s_abs = t_abs[:, BLOCK:, :]
         dur = np.diff(s, axis=2)
         step_len = s[:, 1:, 0] - s[:, :-1, 0]
-        out = {"tuning": {"slot_bytes": slot, "inflight": infl, "dbg": dbg}, "geo": geo,
+        out = {"tuning": {"slot_bytes": slot, "dbg": dbg}, "geo": geo,
                "ms_per_sweep_traced": kms.value / args.sweeps, "ms_per_sweep": float(np.median(ts)),
                "sweeps_per_s": 1e3 / float(np.median(ts)),
                "us_per_block_step": float(step_len.mean()),
@@ -155,18 +154,13 @@ def main():
                 round(float((ft[:, :, 80] - off - fp[:, :, 3]).mean()), 3)
             out["tiles_us"]["pass2 tile 0 landed, after the end of gather D"] = \
                 round(float((ft[:, :, 32] - off - fp[:, :, 7]).mean()), 3)
-            if dbg & 512:
-                out["tiles_us"]["pass2 tile 0 really landed (producer polls), after its issue"] = \
-                    round(float((ft[:, :, 95] - ft[:, :, 80]).mean()), 3)
-                out["tiles_us"]["pass2 tile 0 really landed, after the end of gather D"] = \
-                    round(float((ft[:, :, 95] - off - fp[:, :, 7]).mean()), 3)
             out["tiles_us"]["pass2 tile 0 landed, after its issue"] = round(float((ft[:, :, 32] - ft[:, :, 80]).mean()), 3)
             out["tiles_us"]["pass2 tile end -> next tile start"] = \
                 [round(float((ft[:, :, 32 + t + 1] - ft[:, :, 48 + t]).mean()), 3) for t in range(ntile - 1)]
         results.append(out)
         if args.raw:
-            np.save("%s_%d_%d_%d.npy" % (args.raw, slot, infl, dbg), tr)
-            np.save("%s_tiles_%d_%d_%d.npy" % (args.raw, slot, infl, dbg), tt[::16])
+            np.save("%s_%d_%d.npy" % (args.raw, slot, dbg), tr)
+            np.save("%s_tiles_%d_%d.npy" % (args.raw, slot, dbg), tt[::16])
         if world > 1:
             out["rank"] = rank
         if rank == 0 or args.all_ranks:
