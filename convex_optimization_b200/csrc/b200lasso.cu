@@ -3045,7 +3045,10 @@ static int plan_geometry(b200l_ctx *c) {
     // columns of every block owned by one CTA: a power of two (shift/mask addressing)
     int cs = 1, cs_shift = 0;
     while (cs * G < ld) { cs *= 2; ++cs_shift; }
-    if (cs > MAX_CS) return fail("internal: slice width %d > %d", cs, MAX_CS);
+    if (cs > MAX_CS)
+        return fail("block width w=%d is too wide for the fused kernel: each of the %d CTAs owns at most %d columns "
+                    "of a block, so blocks of up to %d columns (padded) are supported (use more column blocks)",
+                    c->w, G, MAX_CS, G * MAX_CS);
     // the partial gradient goes out straight from registers when every thread holds complete column sums
     // (one row group) and a column group (4 words, two 256-bit stores) fits one message of cs * es / 4 words;
     // otherwise the row groups are combined through shared memory first

@@ -211,8 +211,10 @@ class ClassLasso(ClassLassoCPU):
 
     def _fused_supported(self):
         """the fused kernel has shape limits the reference does not (a row of a block must fit a
-        32 KiB tile, N / #SM <= 1024 fp32 / 512 fp64 entries for the pre-transposed layout); shapes beyond them run the
-        step-wise path on the library's mat-vec kernels instead, with a warning"""
+        32 KiB tile, w <= 64 * #SM, N / #SM <= 1024 fp32 / 512 fp64 entries for the pre-transposed layout, and for the
+        row-major layout N / #SM rows small enough that their buffers leave two tile slots in shared memory: on a B200
+        about 1,500-5,300 rows in fp64 and 2,400-6,700 in fp32 depending on w, INTEGRATION.md section 4); shapes beyond
+        them run the step-wise path on the library's mat-vec kernels instead, with a warning"""
         try:
             self.gpu_cal.run_config()
             return True
